@@ -346,6 +346,32 @@ class Workload:
         self.fe.describe_brief(self.pyr_cur_d, self.d_pri, self.d_desc_t, self.d_val_t, n=n, per_frame=NKP)
         self.fe.describe_brief(self.pyr_cur_d, self.d_new, self.d_desc_n, self.d_val_n, n=B * self.ncell, per_frame=self.ncell)
 
+    def dump_outputs(self, out_dir: str, max_bytes: int = 64 << 20):
+        """Write what the last resident step computed, frame by frame, as float32 DIR/<name>.npy: the tracked keypoints and
+        their status, the adapted FAST thresholds, the new keypoints and their count, and the descriptors of both with their
+        validity flags.  Slots past a frame's new-keypoint count and descriptors flagged invalid hold no result and are written
+        as 0.  A batch whose outputs exceed `max_bytes` is written for a fixed, seeded sample of its frames (frame_index.npy)."""
+        self.torch.cuda.synchronize()
+        B, nc = self.B, self.ncell
+        get = lambda t, *shape: t.cpu().numpy().reshape(B, *shape)
+        out = {"tracked_kps": get(self.d_pri, NKP, 2), "track_status": get(self.d_status, NKP), "fast_threshold": get(self.d_th),
+               "new_kps": get(self.d_new, nc, 2), "new_count": get(self.d_cnt), "tracked_desc": get(self.d_desc_t, NKP, 32),
+               "tracked_desc_valid": get(self.d_val_t, NKP), "new_desc": get(self.d_desc_n, nc, 32), "new_desc_valid": get(self.d_val_n, nc)}
+        empty = np.arange(nc)[None, :] >= out["new_count"][:, None]
+        out["new_kps"][empty] = 0
+        out["new_desc_valid"][empty] = 0
+        out["tracked_desc"][out["tracked_desc_valid"] == 0] = 0
+        out["new_desc"][out["new_desc_valid"] == 0] = 0
+        frame_bytes = 4 * (1 + sum(a[0].size for a in out.values()))
+        frames = np.arange(B)
+        if B * frame_bytes > max_bytes:
+            frames = np.sort(np.random.default_rng(0).choice(B, max_bytes // frame_bytes, replace=False))
+        out = {k: v[frames] for k, v in out.items()}
+        out["frame_index"] = frames
+        os.makedirs(out_dir, exist_ok=True)
+        for k, v in out.items():
+            np.save(os.path.join(out_dir, k + ".npy"), v.astype(np.float32))
+
     # ---- end-to-end arm: the batch is cut into chunks, each chunk goes through the same C-ABI calls
     # with HOST pointers on its own context (= its own stream) from its own host thread, so the
     # H2D/D2H copies of one chunk overlap the kernels of another (the reference itself runs its
@@ -511,6 +537,8 @@ def gpu_arm(args):
     if rank == 0:
         sampler.start()
     ms_res, wall_res, launches = timed(wl.step_resident, args.steps, args.warmup)
+    if args.dump_outputs and rank == 0:
+        wl.dump_outputs(args.dump_outputs)
     if args.kernels_only:
         # profiler runs (ncu serialises kernels; the multi-threaded e2e arm must not run under it)
         if rank == 0:
@@ -819,6 +847,8 @@ def main():
     ap.add_argument("--c4-steps", type=int, default=10)
     ap.add_argument("--c5-reps", type=int, default=5)
     ap.add_argument("--c5-small", action="store_true", help="20 KF x 3000 pts x 18000 obs instead of the C5 window (debugging)")
+    ap.add_argument("--dump-outputs", metavar="DIR", help="write what the last timed front-end step computed to DIR/<name>.npy "
+                                                          "(float32, at most 64 MB; the inputs are the same from run to run)")
     args = ap.parse_args()
     if args.impl == "reference":
         return reference_arm(args)

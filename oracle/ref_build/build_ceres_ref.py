@@ -46,7 +46,7 @@ def available() -> bool:
 
 
 def build(force: bool = False, verbose: bool = False):
-    if not CERES.exists():
+    if not os.access(CERES, os.R_OK):
         return OUT if OUT.exists() else None
     src = sources()
     deps = src + [p for p in (HERE / "mini").rglob("*") if p.is_file()] + [p for p in (HERE / "ceres_cfg").rglob("*") if p.is_file()]

@@ -30,7 +30,7 @@ def available() -> bool:
 
 
 def build(force: bool = False):
-    if not (REF / "src" / "optimizer.cpp").exists():
+    if not os.access(REF / "src" / "optimizer.cpp", os.R_OK):
         return OUT if OUT.exists() else None
     if build_ceres_ref.build() is None:
         return None

@@ -9,6 +9,7 @@ git-ignored, not gpurun-ignored); `build()` returns the existing file when the r
 """
 from __future__ import annotations
 
+import os
 import subprocess
 from pathlib import Path
 
@@ -24,7 +25,7 @@ def available() -> bool:
 
 
 def build(force: bool = False) -> Path | None:
-    if not SRC.exists():
+    if not os.access(SRC, os.R_OK):
         return OUT if OUT.exists() else None
     deps = [SRC, HERE / "residual_ref.cpp"] + [p for p in (HERE / "mini").rglob("*") if p.is_file()]
     if not force and OUT.exists() and all(OUT.stat().st_mtime >= d.stat().st_mtime for d in deps):

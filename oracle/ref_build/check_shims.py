@@ -8,7 +8,7 @@ The two drop-in headers (host/feature_extractor.hpp, host/feature_tracker.hpp) R
 include-path order cannot substitute them.  The check therefore compiles against an overlay directory: links to every reference header
 except those two, which link to the drop-ins.
 
-TEST INFRASTRUCTURE: only tests/ use this."""
+Needs the original project's sources, so it is not part of the test suite: run it as `python -m oracle.ref_build.check_shims`."""
 from __future__ import annotations
 
 import os

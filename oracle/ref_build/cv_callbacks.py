@@ -4,6 +4,7 @@ TEST INFRASTRUCTURE: only tests/ use this."""
 from __future__ import annotations
 
 import ctypes as C
+import os
 import subprocess
 from pathlib import Path
 
@@ -135,7 +136,7 @@ def available() -> bool:
 def build(force: bool = False):
     """oracle/_ref/libov2ref_frontend.so: the reference's src/feature_extractor.cpp and src/feature_tracker.cpp (in place) + fe_ref.cpp, against mini_cv (OpenCV
     containers), the reference tree's Sophus and the stand-in Eigen header."""
-    if not SRC.exists():
+    if not os.access(SRC, os.R_OK):
         return OUT if OUT.exists() else None
     deps = [SRC, SRC2, HERE / "fe_ref.cpp"] + [p for d in ("mini", "mini_cv") for p in (HERE / d).rglob("*") if p.is_file()]
     if not force and OUT.exists() and all(OUT.stat().st_mtime >= d.stat().st_mtime for d in deps):

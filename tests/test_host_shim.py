@@ -595,16 +595,3 @@ def test_clahe_adapter_routes_cv_clahe_calls_to_the_device_call(tmp_path):
         assert tuple(rec[1:3]) == (w, h) and rec[3] == w and rec[4] == 1 and rec[5] == 3000 and tuple(rec[6:8]) == (w // 50, h // 50)
         assert rec[8] == 1          # both calls equalise in place in the destination's layout (the source was copied there first / is it)
 
-
-@pytest.mark.parametrize("shim", ["feature_extractor.cpp", "feature_tracker.cpp", "clahe_gpu.cpp", "optimizer_localba_gpu.cpp", "multi_view_geometry_pnp_gpu.cpp",
-                                  "mapper_match_gpu.cpp", "map_manager_stereo_gpu.cpp"])
-def test_shims_compile_against_the_reference_own_headers(shim):
-    """Every drop-in translation unit against /root/reference/include itself (optimizer.hpp, map_manager.hpp, mapper.hpp, frame.hpp,
-    multi_view_geometry.hpp ...; the two drop-in class headers in place of the reference's feature_extractor.hpp / feature_tracker.hpp),
-    with this container's stand-ins only for the third-party headers it lacks (oracle/ref_build/check_shims.py).  The self-tests above
-    use reduced stand-ins of the map classes; this check is what says the member and method names the shims rely on exist."""
-    from oracle.ref_build import check_shims
-    if not check_shims.available():
-        pytest.skip("/root/reference is not present")
-    err = check_shims.check(shim)
-    assert not err, err[:3000]

@@ -14,6 +14,7 @@ import pytest
 from oracle import ba_ref as B
 from oracle.ref_build import build_ceres_ref
 from ov2slam_b200 import synth
+from reference_calls import library
 
 D, I, U = C.POINTER(C.c_double), C.POINTER(C.c_int32), C.POINTER(C.c_uint8)
 TERM = {0: "CONVERGENCE", 1: "NO_CONVERGENCE", 2: "FAILURE"}
@@ -21,12 +22,12 @@ TERM = {0: "CONVERGENCE", 1: "NO_CONVERGENCE", 2: "FAILURE"}
 
 @pytest.fixture(scope="module")
 def lib():
-    so = build_ceres_ref.build()
-    if so is None:
-        pytest.skip("neither /root/reference nor a prebuilt oracle/_ref is present")
-    lib = C.CDLL(str(so))
-    lib.ov2ref_local_ba.restype = C.c_int
-    return lib
+    def load():
+        so = build_ceres_ref.build()
+        return None if so is None else C.CDLL(str(so))
+    with library("ceres", load) as lib:
+        lib.ov2ref_local_ba.restype = C.c_int
+        yield lib
 
 
 def run_ceres(lib, pb, max_iters_robust=5, max_iters_refine=10, th=5.9915, ftol=1e-3, robust=1, l2=1, maxlog=128):

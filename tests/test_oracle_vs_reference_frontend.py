@@ -12,6 +12,7 @@ import pytest
 
 from oracle import image_ref as R
 from ov2slam_b200 import synth
+from reference_calls import library
 
 cv2 = pytest.importorskip("cv2")
 
@@ -19,10 +20,8 @@ cv2 = pytest.importorskip("cv2")
 @pytest.fixture(scope="module")
 def ref():
     from oracle.ref_build import cv_callbacks as CB
-    lib = CB.load()
-    if lib is None:
-        pytest.skip("neither /root/reference nor a prebuilt oracle/_ref is present")
-    return lib, CB
+    with library("frontend", CB.load) as lib:
+        yield lib, CB
 
 
 def _call(ref, name, fe, im, cs, cur, roi, state_type):

@@ -16,6 +16,7 @@ import pytest
 
 from oracle import ba_ref as B
 from ov2slam_b200 import build, synth
+from reference_calls import library
 
 pytest.importorskip("cv2")
 ROOT = Path(__file__).resolve().parents[1]
@@ -25,14 +26,18 @@ D, I, U = C.POINTER(C.c_double), C.POINTER(C.c_int32), C.POINTER(C.c_uint8)
 @pytest.fixture(scope="module")
 def lib():
     from oracle.ref_build import build_map_ref, cv_callbacks as CB
-    so = build_map_ref.build()
-    if so is None:
-        pytest.skip("neither /root/reference nor a prebuilt oracle/_ref is present")
-    lib = C.CDLL(str(so))
-    cb = CB._Callbacks(*[C.cast(f, C.c_void_p) for f in CB._KEEP])
-    lib.ov2ref_cv_set_callbacks(C.byref(cb))
-    lib.ov2ref_run_local_ba.restype = C.c_int
-    return lib
+
+    def load():
+        so = build_map_ref.build()
+        if so is None:
+            return None
+        lib = C.CDLL(str(so))
+        cb = CB._Callbacks(*[C.cast(f, C.c_void_p) for f in CB._KEEP])
+        lib.ov2ref_cv_set_callbacks(C.byref(cb))
+        return lib
+    with library("map", load) as lib:
+        lib.ov2ref_run_local_ba.restype = C.c_int
+        yield lib
 
 
 def reference_local_ba(lib, pb, nmin_covscore=25, mode=0):

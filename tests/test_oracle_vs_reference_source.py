@@ -11,6 +11,7 @@ import pytest
 from oracle import ba_ref as B
 from oracle import pnp_ref as P
 from oracle.ref_build import build_ref
+from reference_calls import library
 
 K = np.array([458.654, 457.296, 367.215, 248.375])
 KR = np.array([457.587, 456.134, 379.999, 255.238])
@@ -19,13 +20,13 @@ D = C.POINTER(C.c_double)
 
 @pytest.fixture(scope="module")
 def ref():
-    so = build_ref.build()
-    if so is None:
-        pytest.skip("neither /root/reference nor a prebuilt oracle/_ref is present")
-    lib = C.CDLL(str(so))
-    for name in ("ref_eval_anch_invdepth", "ref_eval_right_anch", "ref_eval_right_cam", "ref_eval_pnp", "ref_se3_plus"):
-        getattr(lib, name).restype = C.c_int
-    return lib
+    def load():
+        so = build_ref.build()
+        return None if so is None else C.CDLL(str(so))
+    with library("residuals", load) as lib:
+        for name in ("ref_eval_anch_invdepth", "ref_eval_right_anch", "ref_eval_right_cam", "ref_eval_pnp", "ref_se3_plus"):
+            getattr(lib, name).restype = C.c_int
+        yield lib
 
 
 def p(a):
