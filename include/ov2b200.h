@@ -324,16 +324,32 @@ typedef struct {
     int    termination;                 /* 0 convergence, 1 max iterations, 2 failure */
 } ov2_ba_result;
 
+/* Capacity of one ov2_localba_solve window (the loop closer's looseBA and fullBA hand over windows of hundreds of
+ * keyframes).  Windows of up to OV2_BA_SMALL_MAX_OPT_KEYFRAMES optimised keyframes run the kernel of csrc/ba_lm.cu (or, with
+ * more than OV2_BA_SMALL_MAX_KEYFRAMES keyframes in total, the round-1 path, which has no limit on the total); larger ones the
+ * large-window kernel of csrc/ba_large.cu, whose dense tiled reduced system needs (6 x optimised keyframes)^2 x 8 bytes
+ * (302 MB at the cap) besides ~310 bytes per residual block; a window whose device memory plan exceeds
+ * OV2_BA_LARGE_MAX_BYTES is refused with OV2_ERR_CAPACITY.  ov2_localba_solve_batch, _p2p and _sharded keep the small-window
+ * limits. */
+#define OV2_BA_MAX_OPT_KEYFRAMES       1024
+#define OV2_BA_MAX_KEYFRAMES           4096
+#define OV2_BA_SMALL_MAX_OPT_KEYFRAMES 64
+#define OV2_BA_SMALL_MAX_KEYFRAMES     256
+#define OV2_BA_LARGE_MAX_BYTES         (16ull << 30)
+
 /* outlier_out (optional): [nobs] bytes, bit0 = flagged after solve #1, bit1 = after solve #2.
  * The whole two-stage solve (both Ceres solves, every LM iteration, both outlier scans) is ONE kernel launch with the
- * trust-region controller on the device (csrc/ba_lm.cu); OV2_BA_LEGACY=1 selects the round-1 path (one launch per phase,
- * controller on the host) as a cross-check.  At most 64 optimised and 256 total keyframes per window.
+ * trust-region controller on the device (csrc/ba_lm.cu, csrc/ba_large.cu); OV2_BA_LEGACY=1 selects the round-1 path (one
+ * launch per phase, controller on the host, at most 64 optimised keyframes) as a cross-check.  At most
+ * OV2_BA_MAX_OPT_KEYFRAMES optimised and OV2_BA_MAX_KEYFRAMES total keyframes per window (more: OV2_ERR_CAPACITY), or
+ * at most OV2_BA_SMALL_MAX_OPT_KEYFRAMES optimised keyframes and any total.
  * Residency of a window's arrays is decided on `pose`: host poses = every array of the window (and outlier_out) is host
  * memory, the reference's flow; device poses = each array is inspected and may be either. */
 OV2_API ov2_status ov2_localba_solve(ov2_ctx* ctx, const ov2_ba_problem* pb, const ov2_ba_opts* opts,
                              ov2_ba_result* res, uint8_t* outlier_out);
 
-/* K independent windows in ONE launch (the solves/s metric; SURVEY.md 7 "hard parts" (ii)): window k is pbs[k] with results[k]
+/* K independent windows in ONE launch (the solves/s metric; SURVEY.md 7 "hard parts" (ii)), each of at most 64 optimised and
+ * 256 total keyframes (more: OV2_ERR_CAPACITY): window k is pbs[k] with results[k]
  * and outlier_outs[k] (NULL entries / NULL array allowed); the same options for every window.  Groups of thread blocks pull
  * windows round-robin, every group runs the whole two-stage solve of its window on the device. */
 OV2_API ov2_status ov2_localba_solve_batch(ov2_ctx* ctx, int nprob, const ov2_ba_problem* pbs, const ov2_ba_opts* opts,

@@ -437,6 +437,14 @@ def _stereo_ptrs(pb: dict, keep: dict):
     return keep["obs_type"].ctypes.data, keep["Kr"].ctypes.data, keep["Trl"].ctypes.data
 
 
+# Capacity of one Optimizer.local_ba / ov2_localba_solve window (include/ov2b200.h): optimised and total keyframes.  Windows
+# of up to 64 optimised keyframes run the small-window kernel, larger ones the large-window kernel; batches and the
+# multi-GPU solves keep 64 / 256.
+OV2_BA_MAX_OPT_KEYFRAMES = 1024
+OV2_BA_MAX_KEYFRAMES = 4096
+OV2_BA_SMALL_MAX_OPT_KEYFRAMES = 64
+OV2_BA_SMALL_MAX_KEYFRAMES = 256
+
 DEFAULT_BA_OPTS = dict(max_iters_robust=5, max_iters_refine=10, huber_th=5.9915, function_tolerance=1e-3,
                        use_robust=1, apply_l2_after_robust=1, refine_loss=-1)
 

@@ -32,6 +32,7 @@ SOURCES = {
     "frontend_step.cu": [],
     "ba_solver.cu": [],
     "ba_lm.cu": [],
+    "ba_large.cu": [],
     "ba_comm.cu": [],
     "pnp_solver.cu": [],
     "match_map.cu": ["-fmad=false"],

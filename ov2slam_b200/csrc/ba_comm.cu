@@ -52,11 +52,33 @@ static const int* stop_flag_dev(ov2_ctx* ctx) {
     return d;
 }
 
+static_assert(MAX_VAR_CAMS == OV2_BA_SMALL_MAX_OPT_KEYFRAMES && MAX_CAMS == OV2_BA_SMALL_MAX_KEYFRAMES,
+              "the published small-window limits are ba_lm_kernel's");
+
+// Number of optimised (non-constant) keyframes of a window; pose_const may be device memory when pose is.
+static int optimised_keyframes(const ov2_ba_problem* pb) {
+    if (!pb->pose_const || pb->ncam <= 0) return 0;
+    std::vector<uint8_t> h;
+    const uint8_t* pc = pb->pose_const;
+    if (ov2_is_device_ptr(pb->pose) && ov2_is_device_ptr(pc)) {
+        h.resize(pb->ncam);
+        if (cudaMemcpy(h.data(), pc, pb->ncam, cudaMemcpyDeviceToHost) != cudaSuccess) { cudaGetLastError(); return 0; }
+        pc = h.data();
+    }
+    int ncv = 0;
+    for (int c = 0; c < pb->ncam; ++c) ncv += pc[c] ? 0 : 1;
+    return ncv;
+}
+
 extern "C" ov2_status ov2_localba_solve(ov2_ctx* ctx, const ov2_ba_problem* pb, const ov2_ba_opts* opts,
                                         ov2_ba_result* res, uint8_t* outlier_out) {
     if (!ctx || !pb || !opts || !res) return ov2_fail(ctx, OV2_ERR_INVALID, "ov2_localba_solve: bad arguments");
     const char* e = getenv("OV2_BA_LEGACY");
-    if ((e && atoi(e) != 0) || pb->ncam > MAX_CAMS) return ov2_localba_solve_legacy(ctx, pb, opts, res, outlier_out);
+    const bool legacy = e && atoi(e) != 0;
+    // more than 64 optimised keyframes: the large-window solve (ba_large.cu); smaller windows are routed as before
+    if (!legacy && pb->ncam > MAX_VAR_CAMS && optimised_keyframes(pb) > MAX_VAR_CAMS)
+        return balm_solve_large(ctx, pb, opts, res, outlier_out, stop_flag_dev(ctx));
+    if (legacy || pb->ncam > MAX_CAMS) return ov2_localba_solve_legacy(ctx, pb, opts, res, outlier_out);
     memset(res, 0, sizeof(*res));
     if (pb->nobs == 0) return OV2_OK;
     uint8_t* outs[1] = {outlier_out};

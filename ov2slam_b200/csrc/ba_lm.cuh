@@ -8,7 +8,7 @@ namespace balm {
 
 constexpr unsigned FULL = 0xffffffffu;
 constexpr int THREADS = 256, WARPS = THREADS / 32;
-constexpr int MAX_VAR_CAMS = 64;            // optimised keyframes per window
+constexpr int MAX_VAR_CAMS = 64;            // optimised keyframes per window (ba_lm_kernel; larger windows: ba_large.cu)
 constexpr int MAX_N = 6 * MAX_VAR_CAMS;     // reduced camera system
 constexpr int MAX_CAMS = 256;               // keyframes per window (optimised + constant)
 constexpr int CH_NB = 32;                   // block size of the blocked Cholesky
@@ -75,3 +75,7 @@ struct Peers {
 // Solves `nprob` windows with one launch (peers == NULL: single GPU).  ba_lm.cu
 ov2_status balm_solve(ov2_ctx* ctx, int nprob, const ov2_ba_problem* pbs, const ov2_ba_opts* opts, ov2_ba_result* results,
                       uint8_t* const* outlier_outs, const balm::Peers* peers, const int* stop_flag_dev);
+
+// One window with more than MAX_VAR_CAMS optimised keyframes (up to OV2_BA_MAX_OPT_KEYFRAMES).  ba_large.cu
+ov2_status balm_solve_large(ov2_ctx* ctx, const ov2_ba_problem* pb, const ov2_ba_opts* opts, ov2_ba_result* res,
+                            uint8_t* outlier_out, const int* stop_flag_dev);

@@ -113,7 +113,10 @@ void flatten_landmarks(MapManager& map, Window& win, const std::vector<int>& lm_
 }
 
 // Gauge (at least two constant keyframes in mono, one in stereo: optimizer.cpp:65-69, 396-407 / :1228-1239 / :1992-2003) and the solver's
-// capacity (64 optimised keyframes: beyond that the OLDEST optimised keyframes are held constant, said once on stderr).
+// capacity (OV2_BA_MAX_OPT_KEYFRAMES optimised keyframes: beyond that the OLDEST optimised keyframes are held constant, said once
+// on stderr).  A window of more than OV2_BA_MAX_KEYFRAMES keyframes in total (a fullBA over a very long run) cannot take the
+// large-window solve at all, whatever is held constant: it keeps OV2_BA_SMALL_MAX_OPT_KEYFRAMES (64) optimised keyframes, the
+// window the round-1 solve takes at any total size.
 // `reference_walk` (localBA): the reference walks its keyframe hash map from begin() and counts every keyframe it visits, constant
 // already or not (`nbcstkfs++`, :400-406) - with libstdc++ the walk starts at the LAST keyframe inserted, which is keyframe 0 of a
 // fully covisible window: it is "fixed" a second time, the count reaches two and only ONE keyframe is constant.  The drop-in does the
@@ -133,10 +136,11 @@ void fix_gauge_and_capacity(Window& win, const bool stereo, const char* who, con
             if (!win.pose_const[it->second]) { win.pose_const[it->second] = 1; nconst++; }
     }
     size_t nvar = win.pose_const.size() - nconst;
-    if (nvar > 64) {
+    const size_t cap = win.pose_const.size() > OV2_BA_MAX_KEYFRAMES ? OV2_BA_SMALL_MAX_OPT_KEYFRAMES : OV2_BA_MAX_OPT_KEYFRAMES;
+    if (nvar > cap) {
         static bool told = false;
-        if (!told) { std::cerr << "[ov2b200] " << who << ": " << nvar << " optimised keyframes, the oldest " << nvar - 64 << " are held constant\n"; told = true; }
-        for (auto it = by_id.begin(); nvar > 64 && it != by_id.end(); ++it)
+        if (!told) { std::cerr << "[ov2b200] " << who << ": " << nvar << " optimised keyframes, the oldest " << nvar - cap << " are held constant\n"; told = true; }
+        for (auto it = by_id.begin(); nvar > cap && it != by_id.end(); ++it)
             if (!win.pose_const[it->second]) { win.pose_const[it->second] = 1; nvar--; }
     }
 }

@@ -292,6 +292,133 @@ def make_ba_problem(seed: int, ncam: int = 10, npts: int = 2000, nobs: int = 800
     )
 
 
+def make_loop_ba_problem(seed: int, nkf: int = 160, npts: int = 8000, obs_per_pt: int = 5, outlier_frac: float = 0.05,
+                         px_noise: float = 0.5, w: int = 752, h: int = 480, stereo: bool = False, baseline: float = 0.11,
+                         nconst_extra: int = 0, step: float = 0.2):
+    """A long BA window over a CLOSED trajectory (loop-closure looseBA / fullBA sizes), vectorised, in the conventions of
+    make_ba_problem: anchor = lowest-index observer, observations sorted by landmark (non-anchor views in ascending
+    keyframe order), f32-representable pixels, truth_pose / truth_invdepth, the first 2 (mono) / 1 (stereo) keyframes
+    constant, stereo residual types 2 / 0 / 1 as make_ba_problem lays them out.
+
+    `nkf` keyframes sit on a circle (`step` metres apart) looking outwards; a landmark is seen by `obs_per_pt` + 1
+    consecutive keyframes, so the reduced camera system is a band, and the landmarks around the start are seen by the last
+    keyframes as well: the loop-closure blocks.  `nconst_extra` constant keyframes (a second pass half a step off the first)
+    are appended after the `nkf`; each sees the landmarks in front of it once more (windows with more than 256 keyframes in
+    total)."""
+    rng = np.random.default_rng(seed)
+    fx = fy = 458.654
+    cx, cy = 367.215, 248.375
+    K = np.array([fx, fy, cx, cy])
+    R0 = nkf * step / (2 * np.pi)
+
+    def rig(theta, y):
+        c, s_ = np.cos(theta), np.sin(theta)
+        Rwc = np.zeros((len(theta), 3, 3))
+        Rwc[:, :, 0] = np.stack([s_, np.zeros_like(c), -c], 1)     # x: tangent
+        Rwc[:, 1, 1] = 1.0                                            # y: world y
+        Rwc[:, :, 2] = np.stack([c, np.zeros_like(c), s_], 1)      # z: outwards
+        twc = np.stack([R0 * c, y, R0 * s_], 1)
+        return Rwc, twc
+
+    th = 2 * np.pi * np.arange(nkf) / nkf
+    Rwc, twc = rig(th + np.deg2rad(rng.uniform(-2, 2, nkf)), rng.normal(0, 0.02, nkf))
+    Rx, tx = rig(2 * np.pi * (np.arange(nconst_extra) + 0.5) / max(nconst_extra, 1), np.full(nconst_extra, 0.05))
+    Rall, tall = np.concatenate([Rwc, Rx]), np.concatenate([twc, tx])
+    ncam = nkf + nconst_extra
+
+    def project(ci, pw):                      # ci [M, k], pw [M, 3] -> px [M, k, 2], z [M, k]
+        pc = np.einsum("mkji,mkj->mki", Rall[ci], pw[:, None, :] - tall[ci])
+        z = pc[..., 2]
+        zs = np.where(np.abs(z) > 1e-9, z, 1e-9)
+        return np.stack([fx * pc[..., 0] / zs + cx, fy * pc[..., 1] / zs + cy], -1), z
+
+    def visible(px, z):
+        return (z > 0.5) & (px[..., 0] >= 5) & (px[..., 0] < w - 5) & (px[..., 1] >= 5) & (px[..., 1] < h - 5)
+
+    k = obs_per_pt + 1
+    pws, cams = [], []
+    have = 0
+    while have < npts:
+        m = 2 * (npts - have) + 64
+        c0 = rng.integers(0, nkf, m)
+        run = (c0[:, None] + np.arange(k)[None, :]) % nkf                       # consecutive keyframes (wrapping: loop)
+        mid = run[:, k // 2]
+        pc = np.stack([rng.uniform(-2.5, 2.5, m), rng.uniform(-1.5, 1.5, m), rng.uniform(4.0, 12.0, m)], 1)
+        pw = np.einsum("mij,mj->mi", Rall[mid], pc) + tall[mid]
+        ok = visible(*project(run, pw)).all(1)
+        pws.append(pw[ok]); cams.append(np.sort(run[ok], 1))
+        have += int(ok.sum())
+    pw = np.concatenate(pws)[:npts]
+    sel = np.concatenate(cams)[:npts]
+    anch = sel[:, 0]
+    # anchor pixel rounded to f32 and the landmark put on that bearing (make_ba_problem's convention)
+    pa, za = project(anch[:, None], pw)
+    pa32 = pa[:, 0].astype(np.float32).astype(np.float64)
+    za = za[:, 0]
+    pc_a = np.stack([(pa32[:, 0] - cx) / fx * za, (pa32[:, 1] - cy) / fy * za, za], 1)
+    pw = np.einsum("mij,mj->mi", Rall[anch], pc_a) + tall[anch]
+    obs = sel[:, 1:]
+    if nconst_extra > 0:
+        ang = np.arctan2(pw[:, 2], pw[:, 0]) % (2 * np.pi)
+        ex = nkf + (np.floor(ang / (2 * np.pi) * nconst_extra).astype(np.int64) % nconst_extra)
+        okx = visible(*project(ex[:, None], pw))[:, 0]
+        obs = np.concatenate([obs, np.where(okx, ex, -1)[:, None]], 1)
+    lm = np.repeat(np.arange(npts), obs.shape[1])
+    oc = obs.reshape(-1)
+    keep = oc >= 0
+    lm, oc = lm[keep], oc[keep]
+    px, _ = project(oc[:, None], pw[lm])
+    px = px[:, 0] + rng.normal(0, px_noise, (len(oc), 2))
+
+    def outliers(p):
+        bad = rng.random(len(p)) < outlier_frac
+        ang_ = rng.uniform(0, 2 * np.pi, len(p))
+        r = rng.uniform(10, 50, len(p))
+        return p + bad[:, None] * r[:, None] * np.stack([np.cos(ang_), np.sin(ang_)], 1)
+
+    px = outliers(px).astype(np.float32).astype(np.float64)
+    truth_pose = np.zeros((ncam, 7))
+    truth_pose[:, :3] = tall
+    truth_pose[:, 3:] = np.array([_rot_to_quat_xyzw(R) for R in Rall])
+    pose_const = np.zeros(ncam, np.uint8)
+    pose_const[:1 if stereo else 2] = 1
+    pose_const[nkf:] = 1
+    pose = truth_pose.copy()
+    for i in np.nonzero(pose_const == 0)[0]:
+        dR = _so3_exp(rng.normal(0, np.deg2rad(0.5), size=3))
+        pose[i, :3] = tall[i] + rng.normal(0, 0.01, size=3)
+        pose[i, 3:] = _rot_to_quat_xyzw(dR @ Rall[i])
+    lm_invdepth_true = 1.0 / za
+    lm_invdepth = lm_invdepth_true * (1 + rng.normal(0, 0.05, size=npts))
+    out = dict(K=K, pose=pose, pose_const=pose_const, lm_anchor_cam=anch.astype(np.int32), lm_anchor_px=pa32,
+               lm_invdepth=lm_invdepth, truth_pose=truth_pose, truth_invdepth=lm_invdepth_true)
+    if not stereo:
+        out.update(obs_cam=oc.astype(np.int32), obs_lm=lm.astype(np.int32), obs_px=px)
+        return out
+    # stereo: per landmark [anchor right view (2)], then (left (0), right (1)) for every other view
+    Trl = np.array([-baseline, 0.0, 0.0, 0.0, 0.0, 0.0, 1.0])
+
+    def right_px(pc):
+        pr = pc + Trl[:3]
+        uv = np.stack([fx * pr[:, 0] / pr[:, 2] + cx, fy * pr[:, 1] / pr[:, 2] + cy], 1) + rng.normal(0, px_noise, (len(pc), 2))
+        return outliers(uv).astype(np.float32).astype(np.float64)
+
+    pcam = np.einsum("mji,mj->mi", Rall[oc], pw[lm] - tall[oc])
+    r_other = right_px(pcam)
+    r_anch = right_px(pc_a)
+    cnt = np.bincount(lm, minlength=npts)
+    start = np.concatenate([[0], np.cumsum(1 + 2 * cnt)])[:-1]                  # first row of each landmark
+    j = np.arange(len(lm)) - np.concatenate([[0], np.cumsum(cnt)])[:-1][lm]      # rank of the view within its landmark
+    nob = int((1 + 2 * cnt).sum())
+    o_cam = np.zeros(nob, np.int32); o_lm = np.zeros(nob, np.int32); o_px = np.zeros((nob, 2)); o_ty = np.zeros(nob, np.uint8)
+    o_cam[start] = anch; o_lm[start] = np.arange(npts); o_px[start] = r_anch; o_ty[start] = 2
+    rl = start[lm] + 1 + 2 * j
+    o_cam[rl] = oc; o_lm[rl] = lm; o_px[rl] = px; o_ty[rl] = 0
+    o_cam[rl + 1] = oc; o_lm[rl + 1] = lm; o_px[rl + 1] = r_other; o_ty[rl + 1] = 1
+    out.update(Kr=K.copy(), Trl=Trl, obs_cam=o_cam, obs_lm=o_lm, obs_px=o_px, obs_type=o_ty)
+    return out
+
+
 # ----------------------------------------------------------------------------- local-map matching scene (Mapper::matchToMap)
 def _proj_radtan(P, K, dist):
     x, y = P[:, 0] / P[:, 2], P[:, 1] / P[:, 2]
